@@ -12,6 +12,13 @@ per GPU, 5 frames per id forced => 163 840 samples per utterance; weak scaling).
           H2D of ids and D2H of the PCM inside the timed region
 Timing: CUDA events on the engine's stream, barrier + synchronize on both sides, max over ranks.
 L2 is flushed (256 MiB write) before every timed step.
+
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR
+
+also writes what the last timed `value` step computed, for comparing two builds output for output:
+DIR/pcm.npy (the batch's int16 PCM as float32) and DIR/sample_offsets.npy (float64, utterance b is
+pcm[so[b]:so[b+1]]); under torchrun each rank adds a _rank<r> suffix.  The inputs are seeded, so the
+same arguments give the same inputs on every run.
 """
 from __future__ import annotations
 
@@ -20,6 +27,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -56,7 +64,7 @@ def get_model(name):
     if p:
         return np.fromfile(p, dtype=np.float32), "shipped", p
     blob = binfmt.synthetic_model(seed=11, **binfmt.ARCH[name])
-    p = os.path.join("/tmp", "stts_%s_random_init.bin" % name)
+    p = os.path.join(tempfile.gettempdir(), "stts_%s_random_init_%d.bin" % (name, os.getuid()))   # per user: /tmp may be shared
     blob.tofile(p)
     return blob, "random-init", p
 
@@ -153,6 +161,22 @@ def run_cpu_best(model_file, n_ids, vocab, forced_per_id, cores, reps, warm_reps
     return best[0], best[1], best[2], table
 
 
+DUMP_LIMIT = 64 << 20     # bytes of .npy data per --dump-outputs directory, all ranks together
+
+
+def dump_outputs(d, pcm, sample_offsets, suffix, budget):
+    """Write one step's outputs as DIR/<name><suffix>.npy.  A PCM over `budget` bytes is cut to a fixed,
+    seeded sample of its positions, written as pcm_index (float64) beside the sampled pcm."""
+    os.makedirs(d, exist_ok=True)
+    out = {"sample_offsets": sample_offsets.astype(np.float64), "pcm": pcm.astype(np.float32)}
+    room = budget - out["sample_offsets"].nbytes - 3 * 128      # 128: .npy header
+    if out["pcm"].nbytes > room:
+        idx = np.sort(np.random.default_rng(0).choice(pcm.size, room // 12, replace=False))
+        out["pcm_index"], out["pcm"] = idx.astype(np.float64), out["pcm"][idx]
+    for name, a in out.items():
+        np.save(os.path.join(d, name + suffix + ".npy"), a)
+
+
 def peaks():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
@@ -203,6 +227,7 @@ def main():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak: --batch utterances per GPU; strong: --batch utterances in total, split over the ranks (BASELINE config 5)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the PCM and sample offsets of the last timed step to DIR/*.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
 
@@ -308,6 +333,9 @@ def main():
     launches = E.kernel_launches() - l0
     barrier()
     stage_ms = E.last_timing()
+    if args.dump_outputs:
+        pcm, so = E.fetch(S, args.batch)
+        dump_outputs(args.dump_outputs, pcm, so, "_rank%d" % rank if world > 1 else "", DUMP_LIMIT // world)
 
     # ---- e2e: host buffers through the C ABI ------------------------------------------------------
     h_ids = torch.from_numpy(ids).pin_memory().numpy()

@@ -9,6 +9,7 @@ container header (convertAudioToWavBuf, test/main.cpp:7-65) is byte-identical, t
 (<= 2 LSB on at most 1e-4 of the samples).  The binary is built by __graft_entry__.build() where /root/reference exists and travels
 in summertts_b200/bin/; the model (with its frontend tail) in oracle/_ref/models/."""
 import os
+import struct
 import subprocess
 
 import numpy as np
@@ -48,17 +49,30 @@ def test_reference_demo_program_linked_against_the_engine(native_lib, tmp_path):
 
 def test_wav_container_matches_reference_header(native_lib, tmp_path):
     """summertts_b200/host/wav.hpp (used by the tts_b200 CLI) writes the reference's container byte for byte: same 44-byte header
-    for the same sample count as the reference program's WAV."""
+    for the same sample count as the reference program's WAV.  Without the shipped model, seeded random weights of the same
+    architecture: the header is the reference's with its two size fields (RIFF chunk, data chunk) for this WAV's sample count."""
     ids_cli = os.path.join(ROOT, "summertts_b200", "bin", "tts_b200_ids")
+    assert os.path.exists(ids_cli), "tts_b200_ids is built by __graft_entry__.build()"
     model = _full_model("single_speaker_fast")
-    if not os.path.exists(ids_cli) or model is None:
-        pytest.skip("tts_b200_ids / model did not travel")
     from parity_util import TEST_TXT_IDS
     g = np.load(os.path.join(GOLDEN, "dropin_single_speaker_fast.npz"))
+    want = g["header"].tobytes()
+    shipped = model is not None
+    if not shipped:
+        from summertts_b200 import binfmt
+
+        model = str(tmp_path / "synthetic.bin")
+        binfmt.synthetic_model(seed=11).astype(np.float32).tofile(model)
     idf = tmp_path / "ids.txt"
     idf.write_text(" ".join(str(i) for i in TEST_TXT_IDS) + "\n")
     out = tmp_path / "o.wav"
     r = subprocess.run([ids_cli, "--ids", str(idf), model, str(out)], capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
     wav = out.read_bytes()
-    assert wav[:44] == g["header"].tobytes() and len(wav) == 44 + 2 * g["pcm"].size
+    if shipped:
+        assert len(wav) == 44 + 2 * g["pcm"].size
+    else:
+        n = len(wav) - 44
+        assert n > 0
+        want = want[:4] + struct.pack("<I", n + 36) + want[8:40] + struct.pack("<I", n)
+    assert wav[:44] == want
