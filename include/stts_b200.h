@@ -93,6 +93,26 @@ int stts_batch_fetch(stts_engine* e, int16_t* pcm_out, int64_t cap_samples, int6
  * over the batch); NULL clears.  Used for shape-stable benches and downstream-stage parity. */
 int stts_set_forced_durations(stts_engine* e, const float* w_ceil, int64_t n);
 
+/* ---- seeded sampling (VITS noise_scale / noise_scale_w) ---------------------------------------------------------------------
+ * The reference hard-codes noiseScale = 0 (SynthesizerTrn.cpp:357): the prior is never sampled and the stochastic duration
+ * predictor starts from z = 0, so every utterance gets the one "mean" prosody.  VITS inference exposes two knobs:
+ *   prior:  z_p = m + eps * exp(logs) * noise_scale   (VITS demo default 0.667)
+ *   SDP:    z = eps * noise_scale_w before nn_flip(z, 0), stochastic duration predictor only (demo default 0.8; a model with the
+ *           FixDurationPredictor has no noise input and ignores it)
+ * eps comes from a counter-based Philox4x32-10 keyed by the utterance's 64-bit seed and indexed by position WITHIN the
+ * utterance, so the result does not depend on batching, streaming chunks or the GPU it runs on.  A scale of 0 skips its noise
+ * term entirely: an utterance with both scales 0 is bit-identical to the deterministic default.  Semantics and the exact random
+ * stream: DESIGN.md §12.
+ *
+ * Sampling for the NEXT staged batches (stts_infer_ids / _batch / _batch_into / stts_batch_stage / stts_infer_stream): n
+ * utterances (must equal B of each later batch, else STTS_E_ARG at stage time); noise_scales / noise_scales_w finite, in
+ * [0, 10] (a NULL one = 0 for all); seeds NULL = 0 for all.  n = 0 or both scale arrays NULL clears (deterministic, the
+ * default).  The shim SynthesizerTrn (the reference's API) never samples. */
+int stts_set_sampling(stts_engine* e, int32_t n, const float* noise_scales, const float* noise_scales_w, const uint64_t* seeds);
+/* Host-only (no GPU): the normals the device draws for `seed`; stream 0 = prior [rows = frames][cols = channels],
+ * 1 = SDP [rows = tokens][cols = 2] (column r = eps_r).  out has rows * cols floats. */
+int stts_debug_noise(uint64_t seed, int32_t stream, int64_t rows, int32_t cols, float* out);
+
 /* stts_create with a pre-packed device image on disk (SURVEY.md §8f rank 4; the reference re-parses and copies every weight at every
  * process start, SynthesizerTrn.cpp:91-167 + utils.cpp:8-32).  A missing / stale / foreign image is ignored and rewritten; a
  * matching one (keyed by a hash of the NN section and the library version) supplies every dense conv's packed device representation.
@@ -111,7 +131,8 @@ int stts_infer_stream(stts_engine* e, const int32_t* ids, int32_t n, int32_t sid
 
 /* Stage tensors of utterance 0 of the last run, time-major [rows][cols] float32.
  * which: 0 xx[T][hidden]  1 m[T][inter]  2 logw[T]  3 w_ceil[T]  4 z_p[F][inter]  5 z[F][inter]
- *        6 o[S] (raw float waveform).  Returns a malloc'd buffer in *out (stts_free). */
+ *        6 o[S] (raw float waveform)  7 logs[T][inter] (only computed when the batch sampled the prior, see
+ *        stts_set_sampling).  Returns a malloc'd buffer in *out (stts_free). */
 int stts_debug_fetch(stts_engine* e, int32_t which, float** out, int64_t* rows, int64_t* cols);
 
 /* Enable keeping of stage tensors (off by default; costs memory traffic). */

@@ -9,7 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libstts_b200.so")
 SRCS = ["engine.cu"]
-DEPS = ["engine.cu", "kernels.cuh", "model.hpp", "conv_tc.cuh", "rb_fused.cuh", "pc_fused.cuh", "nb_fused.cuh", "g2p.cuh", "g2p_phases.hpp", os.path.join("..", "..", "include", "stts_b200.h")]
+DEPS = ["engine.cu", "kernels.cuh", "model.hpp", "conv_tc.cuh", "rb_fused.cuh", "pc_fused.cuh", "nb_fused.cuh", "rng.cuh", "g2p.cuh", "g2p_phases.hpp", os.path.join("..", "..", "include", "stts_b200.h")]
 
 
 def _stale() -> bool:

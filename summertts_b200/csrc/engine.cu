@@ -148,7 +148,7 @@ struct stts_engine {
         float *ek = nullptr, *ev = nullptr;
     };
     std::vector<EncL> enc;
-    DConv encProj;
+    DConv encProj, encProjLogs;   // the m / logs halves of TextEncoder's proj
     // fix dp
     DConv dp1, dp2, dpProj, dpCond;
     DLN dpn1, dpn2;
@@ -199,6 +199,12 @@ struct stts_engine {
     float* d_forced = nullptr;
     size_t stageCapTok = 0, stageCapB = 0;
     std::vector<float> forced;
+    // seeded sampling (stts_set_sampling): per-utterance noise_scale / noise_scale_w / seed for the next staged batches; empty =
+    // deterministic.  Staged copies on the device and whether the staged batch samples the prior / the SDP noise at all.
+    std::vector<float> smpNs, smpNsw;
+    std::vector<uint64_t> smpSeed;
+    float* d_ns = nullptr; float* d_nsw = nullptr; unsigned long long* d_seed = nullptr;
+    bool samplePrior = false, sampleSdp = false;
     // last-run results
     int Ft = 0, maxF = 0;
     int64_t St = 0;
@@ -214,7 +220,7 @@ struct stts_engine {
     size_t streamZCap = 0;
     int streamF = 0;
     struct Dbg {
-        float *xx = nullptr, *m = nullptr, *logw = nullptr, *wceil = nullptr, *zp = nullptr, *z = nullptr, *o = nullptr;
+        float *xx = nullptr, *m = nullptr, *logw = nullptr, *wceil = nullptr, *zp = nullptr, *z = nullptr, *o = nullptr, *logs = nullptr;
     } dbg;
     cudaEvent_t ev[7] = {};
     float lastMs[6] = {};
@@ -673,11 +679,14 @@ void stts_engine::build(const Model& M) {
         if (f.c1.k != f.k || f.c2.k != f.k || f.c1.pad != 0 || f.c2.pad != 0) throw Unsupported("FFN conv shape");
         enc.push_back(L);
     }
-    {   // proj: only the m half is live (logs is multiplied by noiseScale == 0, SynthesizerTrn.cpp:357,383)
+    {   // proj: m = the first half; logs = the second half, live only in batches that sample the prior (the reference multiplies
+        // it by noiseScale == 0, SynthesizerTrn.cpp:357,383)
         inter = E.proj.outCh / 2;
         std::vector<int> om(inter);
         for (int i = 0; i < inter; ++i) om[i] = i;
         encProj = make_conv(E.proj, om);
+        for (int i = 0; i < inter; ++i) om[i] = inter + i;
+        encProjLogs = make_conv(E.proj, om);
     }
     // --- duration predictor
     if (durPredType == 1) {
@@ -851,6 +860,8 @@ void stts_engine::stage(int B_, const int32_t* ids, const int32_t* offs, const i
             if (!(ls[u] > 0.f) || !std::isfinite(ls[u]) || ls[u] > 1000.f) throw ArgError("length_scale must be finite, positive and <= 1000");
     for (float w : forced)
         if (!(w >= 0.f) || w > 65536.f) throw ArgError("forced durations must be finite, non-negative and <= 65536 frames");
+    if (!smpNs.empty() && (int)smpNs.size() != B_)
+        throw ArgError("sampling was set for " + std::to_string(smpNs.size()) + " utterances, the batch has " + std::to_string(B_));
     if (offs[0] != 0) throw ArgError("id_offsets[0] must be 0");
     int mt = 0;
     for (int u = 0; u < B_; ++u) {
@@ -875,6 +886,7 @@ void stts_engine::stage(int B_, const int32_t* ids, const int32_t* offs, const i
         re(d_ids, capTok * 4); re(d_forced, capTok * 4);
         re(d_toff, (capB + 1) * 4); re(d_foff, (capB + 1) * 4); re(d_nfr, capB * 4);
         re(d_sids, capB * 4); re(d_ls, capB * 4); re(d_bseg, 2 * 4);
+        re(d_ns, capB * 4); re(d_nsw, capB * 4); re(d_seed, capB * 8);
         stageCapTok = capTok; stageCapB = capB;
     }
     B = B_; Tt = T; maxT = mt;
@@ -892,6 +904,13 @@ void stts_engine::stage(int B_, const int32_t* ids, const int32_t* offs, const i
     if (!forced.empty()) {
         if ((int64_t)forced.size() != T) throw ArgError("forced durations length != total ids of the batch");
         CUDA_CHECK(cudaMemcpyAsync(d_forced, forced.data(), (size_t)T * 4, cudaMemcpyHostToDevice, stream));
+    }
+    samplePrior = std::any_of(smpNs.begin(), smpNs.end(), [](float v) { return v != 0.f; });
+    sampleSdp = durPredType == 0 && std::any_of(smpNsw.begin(), smpNsw.end(), [](float v) { return v != 0.f; });
+    if (samplePrior || sampleSdp) {
+        CUDA_CHECK(cudaMemcpyAsync(d_ns, smpNs.data(), (size_t)B * 4, cudaMemcpyHostToDevice, stream));
+        CUDA_CHECK(cudaMemcpyAsync(d_nsw, smpNsw.data(), (size_t)B * 4, cudaMemcpyHostToDevice, stream));
+        CUDA_CHECK(cudaMemcpyAsync(d_seed, smpSeed.data(), (size_t)B * 8, cudaMemcpyHostToDevice, stream));
     }
     CUDA_CHECK(cudaStreamSynchronize(stream));  // host vectors above go out of scope
 }
@@ -919,7 +938,7 @@ void stts_engine::run() {
         condFloats += (size_t)gin + 64 + (size_t)H + 64 + (size_t)convPre.Cout + 64;
         for (auto& L : flow) if (L.hasCond) condFloats += (size_t)L.cond.Cout + 64;
     }
-    size_t tokFloats = (size_t)Tt * (H * 5 + 3 * H + 2 * ffnW + inter + 3 * dpW + 64 + 8) + (size_t)B * (condFloats + 2 * 64 * ffnW) + 512 * ffnW + 4096;
+    size_t tokFloats = (size_t)Tt * (H * 5 + 3 * H + 2 * ffnW + 2 * inter + 3 * dpW + 64 + 8) + (size_t)B * (condFloats + 2 * 64 * ffnW) + 512 * ffnW + 4096;
     ensure_ws(tokFloats * 4 + (1 << 20));
     ws.reset();
     float* x = ws.get<float>((size_t)Tt * H);
@@ -933,6 +952,7 @@ void stts_engine::run() {
     if (tensor_mode >= 1) encFhP = arena_planes(Tt, B, (int)ffnW);
 #endif
     float* mbuf = ws.get<float>((size_t)Tt * inter);
+    float* logsbuf = samplePrior ? ws.get<float>((size_t)Tt * inter) : nullptr;
     float* logw = ws.get<float>((size_t)Tt);
     float* wceil = ws.get<float>((size_t)Tt);
     int* tokFirst = ws.get<int>((size_t)Tt);
@@ -997,6 +1017,7 @@ void stts_engine::run() {
         add_ln(x1, y, L.n2, x, Tt);
     }
     conv(encProj, x, H, mbuf, inter, tseg, B, maxT);
+    if (samplePrior) conv(encProjLogs, x, H, logsbuf, inter, tseg, B, maxT);
     CUDA_CHECK(cudaEventRecord(ev[1], stream));
     nvtxRangePop(); nvtxRangePushA("stts:duration_predictor");
 
@@ -1025,8 +1046,13 @@ void stts_engine::run() {
         dds_forward(sdpConvs, d1, d2, d3, tseg, B, maxT, Tt);  // convs
         conv(sdpProj, d1, H, d2, H, tseg, B, maxT);            // XX = proj(...)  -> d2
         float* XX = d2;
-        CUDA_CHECK(cudaMemsetAsync(sa, 0, (size_t)Tt * 4, stream));
-        CUDA_CHECK(cudaMemsetAsync(sb, 0, (size_t)Tt * 4, stream));
+        if (sampleSdp) {
+            sdp_noise_kernel<<<dim3((maxT + 127) / 128, B), 128, 0, stream>>>(sa, sb, d_toff, d_nsw, d_seed);
+            launch_check();
+        } else {
+            CUDA_CHECK(cudaMemsetAsync(sa, 0, (size_t)Tt * 4, stream));
+            CUDA_CHECK(cudaMemsetAsync(sb, 0, (size_t)Tt * 4, stream));
+        }
         float *a = sa, *b = sb;  // (row0, row1) of flapZ_T
         for (int i = sdpNFlows - 1; i > 0; --i) {
             DConvFlow& cf = sdpFlows[i];
@@ -1105,7 +1131,7 @@ void stts_engine::run() {
         CUDA_CHECK(cudaMemcpy(nb, ws.base, tokEnd, cudaMemcpyDeviceToDevice));
         const ptrdiff_t delta = (char*)nb - ws.base;
         auto mv = [&](auto*& p) { if (p) p = (std::remove_reference_t<decltype(p)>)((char*)p + delta); };
-        mv(x); mv(mbuf); mv(logw); mv(wceil); mv(tokFirst); mv(G); mv(gDp); mv(gDec);
+        mv(x); mv(mbuf); mv(logsbuf); mv(logw); mv(wceil); mv(tokFirst); mv(G); mv(gDp); mv(gDec);
         for (auto& g : gWn) mv(g);
         CUDA_CHECK(cudaFree(wsAlloc));
         wsAlloc = nb; ws.base = (char*)nb; ws.cap = want;
@@ -1148,7 +1174,10 @@ void stts_engine::run() {
     if (injectZ) CUDA_CHECK(cudaMemcpyAsync(z, injectZ, (size_t)Ft * inter * 4, cudaMemcpyDeviceToDevice, stream));
     else {
         dim3 g((maxF + 3) / 4, B);
-        regulate_kernel<<<g, 128, 0, stream>>>(mbuf, inter, tokFirst, wceil, d_toff, d_foff, z, inter);
+        if (samplePrior)
+            regulate_noise_kernel<<<g, 128, 0, stream>>>(mbuf, logsbuf, inter, tokFirst, wceil, d_toff, d_foff, z, inter, d_ns, d_seed);
+        else
+            regulate_kernel<<<g, 128, 0, stream>>>(mbuf, inter, tokFirst, wceil, d_toff, d_foff, z, inter);
         launch_check();
         if (debug) CUDA_CHECK(cudaMemcpyAsync(zp_dbg, z, (size_t)Ft * inter * 4, cudaMemcpyDeviceToDevice, stream));
     }
@@ -1493,7 +1522,7 @@ void stts_engine::run() {
     const int sMul = R * tailMul;
     h_soff.assign(B + 1, 0);
     for (int u = 0; u <= B; ++u) h_soff[u] = (int64_t)h_foff[u] * sMul;
-    if (!injectZ) { dbg.xx = x; dbg.m = mbuf; dbg.logw = logw; dbg.wceil = wceil; dbg.zp = zp_dbg; }
+    if (!injectZ) { dbg.xx = x; dbg.m = mbuf; dbg.logs = logsbuf; dbg.logw = logw; dbg.wceil = wceil; dbg.zp = zp_dbg; }
     dbg.z = z; dbg.o = o;
     runValid = true;
 }
@@ -1519,9 +1548,9 @@ extern "C" {
 const char* stts_last_error(void) { return g_last_error.c_str(); }
 const char* stts_version(void) {
 #ifdef STTS_WITH_TC
-    return "stts_b200 0.1 (sm_100a; fp32 FFMA tiles + tcgen05 split-fp16 tiles)";
+    return "stts_b200 0.2 (sm_100a; fp32 FFMA tiles + tcgen05 split-fp16 tiles)";
 #else
-    return "stts_b200 0.1 (sm_100a; fp32 FFMA tiles)";
+    return "stts_b200 0.2 (sm_100a; fp32 FFMA tiles)";
 #endif
 }
 void stts_free(void* p) { free(p); }
@@ -1646,7 +1675,7 @@ void stts_destroy(stts_engine* e) {
     if (e->wsAlloc) cudaFree(e->wsAlloc);
     if (e->streamZ) cudaFree(e->streamZ);
     for (void* p : {(void*)e->d_ids, (void*)e->d_toff, (void*)e->d_sids, (void*)e->d_ls, (void*)e->d_foff, (void*)e->d_nfr,
-                    (void*)e->d_bseg, (void*)e->d_forced})
+                    (void*)e->d_bseg, (void*)e->d_forced, (void*)e->d_ns, (void*)e->d_nsw, (void*)e->d_seed})
         if (p) cudaFree(p);
     if (e->hostPcm) cudaFreeHost(e->hostPcm);
     if (e->hostInts) cudaFreeHost(e->hostInts);
@@ -1683,6 +1712,43 @@ int stts_set_forced_durations(stts_engine* e, const float* w, int64_t n) {
         if (!e) throw ArgError("null engine");
         if (!w || n <= 0) e->forced.clear();
         else e->forced.assign(w, w + n);
+    });
+}
+int stts_set_sampling(stts_engine* e, int32_t n, const float* ns, const float* nsw, const uint64_t* seeds) {
+    return guard([&] {
+        if (!e || n < 0) throw ArgError("null engine or n < 0");
+        if (n == 0 || (!ns && !nsw)) {
+            e->smpNs.clear(); e->smpNsw.clear(); e->smpSeed.clear();
+            return;
+        }
+        std::vector<float> a(n, 0.f), b(n, 0.f);
+        std::vector<uint64_t> s(n, 0);
+        for (int i = 0; i < n; ++i) {
+            if (ns) a[i] = ns[i];
+            if (nsw) b[i] = nsw[i];
+            if (seeds) s[i] = seeds[i];
+            if (!(a[i] >= 0.f && a[i] <= 10.f) || !(b[i] >= 0.f && b[i] <= 10.f))
+                throw ArgError("noise scales must be finite and in [0, 10] (utterance " + std::to_string(i) + ")");
+        }
+        e->smpNs.swap(a); e->smpNsw.swap(b); e->smpSeed.swap(s);
+    });
+}
+int stts_debug_noise(uint64_t seed, int32_t stream, int64_t rows, int32_t cols, float* out) {
+    return guard([&] {
+        if (!out || rows < 0 || cols < 1 || (stream == RNG_STREAM_SDP && cols != 2) || (stream != RNG_STREAM_PRIOR && stream != RNG_STREAM_SDP))
+            throw ArgError("stream 0 (prior, cols >= 1) or 1 (SDP, cols == 2), rows >= 0, out non-null");
+        float e[4];
+        for (int64_t r = 0; r < rows; ++r) {
+            if (stream == RNG_STREAM_SDP) {
+                philox_normals4((uint32_t)r, 0u, 1u, 0u, seed, e);
+                out[r * 2] = e[0]; out[r * 2 + 1] = e[1];
+                continue;
+            }
+            for (int q = 0; 4 * q < cols; ++q) {
+                philox_normals4((uint32_t)r, (uint32_t)q, 0u, 0u, seed, e);
+                for (int j = 0; j < 4 && 4 * q + j < cols; ++j) out[r * cols + 4 * q + j] = e[j];
+            }
+        }
     });
 }
 int stts_debug_enable(stts_engine* e, int32_t on) {
@@ -1845,6 +1911,7 @@ int stts_debug_fetch(stts_engine* e, int32_t which, float** out, int64_t* rows, 
             case 4: src = e->dbg.zp; r = F0; c = e->inter; if (!src) throw ArgError("z_p is only kept when stts_debug_enable(1) was set before the run"); break;
             case 5: src = e->dbg.z; r = F0; c = e->inter; break;
             case 6: src = e->dbg.o; r = e->h_soff[1] - e->h_soff[0]; break;
+            case 7: src = e->dbg.logs; r = T0; c = e->inter; if (!src) throw ArgError("logs is only computed when the batch samples the prior"); break;
             default: throw ArgError("unknown stage id");
         }
         *out = (float*)malloc(std::max<int64_t>(r * c, 1) * 4);

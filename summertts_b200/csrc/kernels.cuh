@@ -13,6 +13,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "rng.cuh"
+
 namespace stts {
 
 // ----------------------------------------------------------------------------------------------
@@ -665,8 +667,21 @@ __global__ void __launch_bounds__(256) durations_kernel(const float* __restrict_
 // ----------------------------------------------------------------------------------------------
 // K9. Length regulator: z_p[f] = m[token(f)]  (row repeat).  expandM, SynthesizerTrn.cpp:304-321,
 // and z_p = m_expand (+ randn*exp(logs)*0), :383 — the RNG term is multiplied by noiseScale == 0
-// (:357) and is not generated.
+// (:357) and is not generated.  (regulate_noise_kernel below generates it for batches that sample.)
 // ----------------------------------------------------------------------------------------------
+// last token of utterance [t0, t0+n) whose first frame <= f, and whether f lies inside it (false on the padding frame of
+// an all-zero-duration utterance)
+__device__ __forceinline__ int regulate_token(const int* __restrict__ tok_first, const float* __restrict__ w_ceil, int t0, int n,
+                                              int f, bool& valid) {
+    int lo = 0, hi = n - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (tok_first[t0 + mid] <= f) lo = mid; else hi = mid - 1;
+    }
+    valid = f < tok_first[t0 + lo] + (int)w_ceil[t0 + lo];
+    return lo;
+}
+
 __global__ void regulate_kernel(const float* __restrict__ m, int ldm, const int* __restrict__ tok_first,
                                 const float* __restrict__ w_ceil, const int* __restrict__ toff,
                                 const int* __restrict__ foff, float* __restrict__ zp, int C) {
@@ -676,16 +691,67 @@ __global__ void regulate_kernel(const float* __restrict__ m, int ldm, const int*
     const int F = foff[u + 1] - foff[u];
     if (f >= F) return;
     const int t0 = toff[u], n = toff[u + 1] - t0;
-    // last token whose first frame <= f
-    int lo = 0, hi = n - 1;
-    while (lo < hi) {
-        const int mid = (lo + hi + 1) >> 1;
-        if (tok_first[t0 + mid] <= f) lo = mid; else hi = mid - 1;
-    }
-    const bool valid = f < tok_first[t0 + lo] + (int)w_ceil[t0 + lo];
+    bool valid;
+    const int lo = regulate_token(tok_first, w_ceil, t0, n, f, valid);
     float* dst = zp + (size_t)(foff[u] + f) * C;
     const float* src = m + (size_t)(t0 + lo) * ldm;
     for (int c = lane; c < C; c += 32) dst[c] = valid ? src[c] : 0.f;
+}
+
+// K9s. Length regulator with the prior sampled (VITS SynthesizerTrn.infer): z_p = m + eps * exp(logs) * noise_scale, on the
+// per-frame m / logs rows of expandM (both 0 on a padding frame, so z_p = eps * noise_scale there).  Same grid as
+// regulate_kernel (one warp per frame); each lane draws one Philox call per channel quad q (counter (f, q, 0, 0), key = the
+// utterance's seed, rng.cuh) and applies exp(logs) in registers, so no eps tensor exists in HBM.  An utterance with
+// noise_scale == 0 copies m exactly as regulate_kernel does: the noise term is skipped, not multiplied (inf * 0 = NaN).
+__global__ void __launch_bounds__(128) regulate_noise_kernel(const float* __restrict__ m, const float* __restrict__ logs, int ldm,
+                                                             const int* __restrict__ tok_first, const float* __restrict__ w_ceil,
+                                                             const int* __restrict__ toff, const int* __restrict__ foff,
+                                                             float* __restrict__ zp, int C, const float* __restrict__ noise_scale,
+                                                             const unsigned long long* __restrict__ seed) {
+    const int u = blockIdx.y;
+    const int f = blockIdx.x * 4 + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    const int F = foff[u + 1] - foff[u];
+    if (f >= F) return;
+    const int t0 = toff[u], n = toff[u + 1] - t0;
+    bool valid;
+    const int lo = regulate_token(tok_first, w_ceil, t0, n, f, valid);
+    float* dst = zp + (size_t)(foff[u] + f) * C;
+    const float* src = m + (size_t)(t0 + lo) * ldm;
+    const float ns = noise_scale[u];
+    if (ns == 0.f) {
+        for (int c = lane; c < C; c += 32) dst[c] = valid ? src[c] : 0.f;
+        return;
+    }
+    const float* ls = logs + (size_t)(t0 + lo) * ldm;
+    const uint64_t key = seed[u];
+    for (int q = lane; 4 * q < C; q += 32) {
+        float e[4];
+        philox_normals4((uint32_t)f, (uint32_t)q, 0u, 0u, key, e);
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const int c = 4 * q + j;
+            if (c < C) dst[c] = valid ? src[c] + e[j] * expf(ls[c]) * ns : e[j] * ns;
+        }
+    }
+}
+
+// K9d. Initial rows of the stochastic duration predictor with noise (VITS: z = randn(2, T) * noise_scale_w, then nn_flip(z, 0),
+// StochasticDurationPredictor.cpp:117-149): eps_r(t) from counter (t, 0, 1, 0) of the utterance's seed.  The flip swaps the two
+// rows, so row 0 of the flipped z (`a`) is eps_1 * noise_scale_w and row 1 (`b`) is eps_0 * noise_scale_w.  noise_scale_w == 0
+// writes exact zeros.  Grid (ceil(maxT / 128), B).
+__global__ void __launch_bounds__(128) sdp_noise_kernel(float* __restrict__ a, float* __restrict__ b, const int* __restrict__ toff,
+                                                        const float* __restrict__ noise_scale_w,
+                                                        const unsigned long long* __restrict__ seed) {
+    const int u = blockIdx.y;
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    const int t0 = toff[u];
+    if (t >= toff[u + 1] - t0) return;
+    const float s = noise_scale_w[u];
+    float e[4] = {0.f, 0.f, 0.f, 0.f};
+    if (s != 0.f) philox_normals4((uint32_t)t, 0u, 1u, 0u, seed[u], e);
+    a[t0 + t] = s != 0.f ? e[1] * s : 0.f;
+    b[t0 + t] = s != 0.f ? e[0] * s : 0.f;
 }
 
 // gather speaker embedding rows: G[u][c] = emg(sid_u, c); emg col-major (spk x gin). SynthesizerTrn.cpp:363-372

@@ -11,6 +11,7 @@ if the library or a B200 is missing, construction raises.
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
 import os
 
@@ -28,6 +29,7 @@ ABI_SYMBOLS = [
     "stts_describe_model", "stts_version", "stts_profile_enable", "stts_profile_fetch",
     "stts_test_conv1d", "stts_debug_pack_weights", "stts_test_rbpair", "stts_tensor_fallbacks", "stts_infer_stream", "stts_create_cached",
     "stts_g2p_create", "stts_g2p_destroy", "stts_g2p_dim", "stts_g2p_predict", "stts_g2p_kernel_launches",
+    "stts_set_sampling", "stts_debug_noise",
 ]
 
 STTS_OK, STTS_E_ARG, STTS_E_FORMAT, STTS_E_UNSUPPORTED, STTS_E_CUDA, STTS_E_NOMEM = 0, -1, -2, -3, -4, -5   # include/stts_b200.h
@@ -67,6 +69,8 @@ def load_library():
     L.stts_batch_run.argtypes = [vp, C.POINTER(i64)]
     L.stts_batch_fetch.argtypes = [vp, vp, i64, vp]
     L.stts_set_forced_durations.argtypes = [vp, vp, i64]
+    L.stts_set_sampling.argtypes = [vp, i32, vp, vp, vp]
+    L.stts_debug_noise.argtypes = [C.c_uint64, i32, i64, i32, vp]
     L.stts_debug_fetch.argtypes = [vp, i32, C.POINTER(vp), C.POINTER(i64), C.POINTER(i64)]
     L.stts_debug_enable.argtypes = [vp, i32]
     L.stts_last_timing.argtypes = [vp, vp, i32]
@@ -107,7 +111,16 @@ def describe_model(blob: np.ndarray):
     return s, end.value
 
 
-STAGES = {"xx": 0, "m": 1, "logw": 2, "w_ceil": 3, "z_p": 4, "z": 5, "o": 6}
+def debug_noise(seed: int, stream: int, rows: int, cols: int = 2) -> np.ndarray:
+    """Host-only: the normals the device draws for `seed` (stts_debug_noise); stream 0 = prior [frames][channels],
+    1 = stochastic duration predictor [tokens][2]."""
+    L = load_library()
+    out = np.empty((rows, cols), np.float32)
+    _check(L.stts_debug_noise(int(seed) & (2 ** 64 - 1), int(stream), int(rows), int(cols), out.ctypes.data))
+    return out
+
+
+STAGES = {"xx": 0, "m": 1, "logw": 2, "w_ceil": 3, "z_p": 4, "z": 5, "o": 6, "logs": 7}
 
 
 class SynthesizerTrn:
@@ -138,12 +151,14 @@ class SynthesizerTrn:
         n = self._L.stts_speaker_num(self._h)
         return 1 if n == 0 else n  # SynthesizerTrn.cpp:83-86
 
-    def infer_ids(self, ids, sid: int = 0, length_scale: float = 1.0) -> np.ndarray:
-        """NN half of SynthesizerTrn::infer for one utterance; returns int16 PCM."""
+    def infer_ids(self, ids, sid: int = 0, length_scale: float = 1.0, noise_scale=0.0, noise_scale_w=0.0, seed=0) -> np.ndarray:
+        """NN half of SynthesizerTrn::infer for one utterance; returns int16 PCM.  noise_scale / noise_scale_w / seed: seeded
+        sampling (set_sampling); the defaults give the reference's deterministic output."""
         ids = np.ascontiguousarray(ids, dtype=np.int32)
         p, n = C.c_void_p(), C.c_int32()
-        _check(self._L.stts_infer_ids(self._h, ids.ctypes.data, ids.size, int(sid), float(length_scale),
-                                      C.byref(p), C.byref(n)))
+        with self._sampling(1, noise_scale, noise_scale_w, seed):
+            _check(self._L.stts_infer_ids(self._h, ids.ctypes.data, ids.size, int(sid), float(length_scale),
+                                          C.byref(p), C.byref(n)))
         out = np.ctypeslib.as_array(C.cast(p, C.POINTER(C.c_int16)), shape=(max(n.value, 1),))[:n.value].copy()
         self._L.stts_free(p)
         return out
@@ -156,17 +171,19 @@ class SynthesizerTrn:
         ids = np.ascontiguousarray(np.concatenate([np.asarray(x, dtype=np.int32) for x in id_lists]), dtype=np.int32)
         return ids, offs
 
-    def infer_batch(self, id_lists, sids=None, length_scales=None):
-        """B utterances -> list of int16 arrays (host buffers in, host buffers out)."""
+    def infer_batch(self, id_lists, sids=None, length_scales=None, noise_scale=0.0, noise_scale_w=0.0, seed=0):
+        """B utterances -> list of int16 arrays (host buffers in, host buffers out).  noise_scale / noise_scale_w / seed:
+        scalars or per-utterance arrays (set_sampling)."""
         ids, offs = self._pack(id_lists)
         B = len(id_lists)
         s = None if sids is None else np.ascontiguousarray(sids, dtype=np.int32)
         ls = None if length_scales is None else np.ascontiguousarray(length_scales, dtype=np.float32)
         ptrs = (C.c_void_p * B)()
         ns = (C.c_int32 * B)()
-        _check(self._L.stts_infer_batch(self._h, B, ids.ctypes.data, offs.ctypes.data,
-                                        None if s is None else s.ctypes.data, None if ls is None else ls.ctypes.data,
-                                        ptrs, ns))
+        with self._sampling(B, noise_scale, noise_scale_w, seed):
+            _check(self._L.stts_infer_batch(self._h, B, ids.ctypes.data, offs.ctypes.data,
+                                            None if s is None else s.ctypes.data, None if ls is None else ls.ctypes.data,
+                                            ptrs, ns))
         outs = []
         for b in range(B):
             a = np.ctypeslib.as_array(C.cast(ptrs[b], C.POINTER(C.c_int16)), shape=(max(ns[b], 1),))[:ns[b]].copy()
@@ -181,12 +198,13 @@ class SynthesizerTrn:
             None if sids is None else sids.ctypes.data, None if length_scales is None else length_scales.ctypes.data,
             pcm_out.ctypes.data, pcm_out.size, sample_offsets.ctypes.data))
 
-    def stage(self, id_lists, sids=None, length_scales=None):
+    def stage(self, id_lists, sids=None, length_scales=None, noise_scale=0.0, noise_scale_w=0.0, seed=0):
         ids, offs = self._pack(id_lists)
         s = None if sids is None else np.ascontiguousarray(sids, dtype=np.int32)
         ls = None if length_scales is None else np.ascontiguousarray(length_scales, dtype=np.float32)
-        _check(self._L.stts_batch_stage(self._h, len(id_lists), ids.ctypes.data, offs.ctypes.data,
-                                        None if s is None else s.ctypes.data, None if ls is None else ls.ctypes.data))
+        with self._sampling(len(id_lists), noise_scale, noise_scale_w, seed):
+            _check(self._L.stts_batch_stage(self._h, len(id_lists), ids.ctypes.data, offs.ctypes.data,
+                                            None if s is None else s.ctypes.data, None if ls is None else ls.ctypes.data))
 
     def run(self) -> int:
         tot = C.c_int64()
@@ -198,6 +216,35 @@ class SynthesizerTrn:
         so = np.zeros(B + 1, dtype=np.int64)
         _check(self._L.stts_batch_fetch(self._h, pcm.ctypes.data, pcm.size, so.ctypes.data))
         return pcm[:total], so
+
+    # -- seeded sampling ---------------------------------------------------------------------------
+    def set_sampling(self, noise_scales=None, noise_scales_w=None, seeds=None):
+        """stts_set_sampling for the next staged batches: per-utterance arrays (their length must equal each later batch's
+        size); None for both scales clears (deterministic, the default)."""
+        if noise_scales is None and noise_scales_w is None:
+            _check(self._L.stts_set_sampling(self._h, 0, None, None, None))
+            return
+        arrs = [None if a is None else np.ascontiguousarray(np.atleast_1d(a), dtype=dt)
+                for a, dt in ((noise_scales, np.float32), (noise_scales_w, np.float32), (seeds, np.uint64))]
+        n = max(a.size for a in arrs if a is not None)
+        if any(a is not None and a.size != n for a in arrs):
+            raise ValueError("noise_scales, noise_scales_w and seeds must have the same length")
+        _check(self._L.stts_set_sampling(self._h, n, *[None if a is None else a.ctypes.data for a in arrs]))
+
+    @contextlib.contextmanager
+    def _sampling(self, B, noise_scale, noise_scale_w, seed):
+        """Per-call sampling of the keyword forms: scalars are broadcast to the B utterances; set before the call and cleared
+        after it.  All-zero scales leave the engine's sampling state alone (the deterministic path)."""
+        if not (np.any(np.asarray(noise_scale) != 0) or np.any(np.asarray(noise_scale_w) != 0)):
+            yield
+            return
+        seeds = np.broadcast_to(np.asarray(seed, dtype=np.uint64), (B,))
+        self.set_sampling(np.broadcast_to(np.asarray(noise_scale, np.float32), (B,)),
+                          np.broadcast_to(np.asarray(noise_scale_w, np.float32), (B,)), seeds)
+        try:
+            yield
+        finally:
+            self.set_sampling(None)
 
     # -- test hooks --------------------------------------------------------------------------------
     def set_forced_durations(self, w):
@@ -237,8 +284,9 @@ class SynthesizerTrn:
     def kernel_launches(self) -> int:
         return int(self._L.stts_kernel_launches(self._h))
 
-    def infer_stream(self, ids, sid=0, length_scale=1.0, chunk_frames=128):
-        """Chunked synthesis: returns (list of per-chunk int16 arrays in emission order, GPU ms to the first chunk)."""
+    def infer_stream(self, ids, sid=0, length_scale=1.0, chunk_frames=128, noise_scale=0.0, noise_scale_w=0.0, seed=0):
+        """Chunked synthesis: returns (list of per-chunk int16 arrays in emission order, GPU ms to the first chunk).  With the
+        same seed and scales, the chunks concatenate to the one-shot infer_ids result."""
         ids = np.ascontiguousarray(ids, dtype=np.int32)
         chunks = []
         CB = C.CFUNCTYPE(None, C.POINTER(C.c_int16), C.c_int64, C.c_void_p)
@@ -250,8 +298,9 @@ class SynthesizerTrn:
         first, total = C.c_float(0), C.c_int64(0)
         self._L.stts_infer_stream.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_float, C.c_int32, CB, C.c_void_p,
                                               C.POINTER(C.c_float), C.POINTER(C.c_int64)]
-        _check(self._L.stts_infer_stream(self._h, ids.ctypes.data, ids.size, int(sid), float(length_scale), int(chunk_frames), cb, None,
-                                         C.byref(first), C.byref(total)))
+        with self._sampling(1, noise_scale, noise_scale_w, seed):
+            _check(self._L.stts_infer_stream(self._h, ids.ctypes.data, ids.size, int(sid), float(length_scale), int(chunk_frames), cb,
+                                             None, C.byref(first), C.byref(total)))
         assert total.value == sum(c.size for c in chunks)
         return chunks, float(first.value)
 

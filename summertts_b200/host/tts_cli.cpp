@@ -12,7 +12,10 @@
 //            --frontend-threads T (text -> ids on T host threads, one frontend instance each: at batch 64 the 3-4 ms/sentence
 //            host frontend, not the GPU, is the serial bottleneck -- SURVEY §8f rank 3), --dump-ids (frontend only: print the
 //            phoneme ids of every utterance, one line each, and stop -- no GPU needed; feeds `--ids` elsewhere),
-//            --selftest-wav <out.wav> (writes one second of a 440 Hz tone; container check without a GPU)
+//            --selftest-wav <out.wav> (writes one second of a 440 Hz tone; container check without a GPU),
+//            --noise-scale NS, --noise-scale-w NSW, --seed S (VITS sampling, stts_set_sampling; defaults 0 0 0 = the reference's
+//            deterministic output): job j of the input -- the j-th non-empty line under --per-line / --ids, the j-th speaker job
+//            of the multi-speaker loop -- gets seed S + j, whatever GPU it lands on
 //
 // Text input needs the host frontend (frontend.hpp; built with -DSTTS_WITH_REF_FRONTEND against the reference's sources by
 // `make REF=...`); the ids-only build has no dependency outside this repository.  No CPU fallback: without a usable
@@ -44,6 +47,8 @@ struct Args {
     bool ids = false, per_line = false, concat = false, dump_ids = false;
     int gpus = 1, sid = -1, fe_threads = 0;
     float length_scale = -1.f;
+    float noise_scale = 0.f, noise_scale_w = 0.f;
+    uint64_t seed = 0;
 };
 
 struct Utt {
@@ -51,6 +56,7 @@ struct Utt {
     std::vector<int32_t> ids;
     float ls = 1.f;
     int32_t sid = 0;
+    uint64_t seed = 0;
     std::string out;
     std::vector<int16_t> pcm;
 };
@@ -58,7 +64,7 @@ struct Utt {
 int usage(const char* argv0) {
     fprintf(stderr,
             "usage: %s [--ids] [--per-line] [--concat] [--dump-ids] [--gpus N] [--frontend-threads T] [--sid S] [--length-scale L]\n"
-            "          <input.txt> <model.bin> <out.wav>\n"
+            "          [--noise-scale NS] [--noise-scale-w NSW] [--seed S] <input.txt> <model.bin> <out.wav>\n"
             "       %s --selftest-wav <out.wav>\n", argv0, argv0);
     return 2;
 }
@@ -92,7 +98,7 @@ std::string numbered(const std::string& out, const char* fmt, int i) {
 }
 
 // one engine per GPU; utterances partitioned longest-first (summertts_b200/shard.py::balanced does the same for Python callers)
-int run_device(int dev, const std::vector<char>& model, std::vector<Utt*>& work, std::string* err) {
+int run_device(int dev, const std::vector<char>& model, std::vector<Utt*>& work, float noise_scale, float noise_scale_w, std::string* err) {
     if (work.empty()) return 0;
     stts_engine* e = nullptr;
     if (stts_create(reinterpret_cast<const float*>(model.data()), (int64_t)model.size(), dev, &e) != STTS_OK) {
@@ -108,9 +114,19 @@ int run_device(int dev, const std::vector<char>& model, std::vector<Utt*>& work,
         offs.push_back((int32_t)ids.size());
         sids[b] = work[b]->sid; ls[b] = work[b]->ls;
     }
-    int rc = stts_infer_batch(e, B, ids.data(), offs.data(), sids.data(), ls.data(), pcm.data(), ns.data());
-    if (rc != STTS_OK) *err = std::string("stts_infer_batch(device ") + std::to_string(dev) + "): " + stts_last_error();
-    else
+    int rc = STTS_OK;
+    if (noise_scale != 0.f || noise_scale_w != 0.f) {
+        std::vector<float> nsv(B, noise_scale), nswv(B, noise_scale_w);
+        std::vector<uint64_t> seeds(B);
+        for (int b = 0; b < B; ++b) seeds[b] = work[b]->seed;
+        rc = stts_set_sampling(e, B, nsv.data(), nswv.data(), seeds.data());
+        if (rc != STTS_OK) *err = std::string("stts_set_sampling: ") + stts_last_error();
+    }
+    if (rc == STTS_OK) {
+        rc = stts_infer_batch(e, B, ids.data(), offs.data(), sids.data(), ls.data(), pcm.data(), ns.data());
+        if (rc != STTS_OK) *err = std::string("stts_infer_batch(device ") + std::to_string(dev) + "): " + stts_last_error();
+    }
+    if (rc == STTS_OK)
         for (int b = 0; b < B; ++b) {
             work[b]->pcm.assign(pcm[b], pcm[b] + ns[b]);
             stts_free(pcm[b]);
@@ -138,6 +154,9 @@ int main(int argc, char** argv) {
         else if (s == "--frontend-threads") a.fe_threads = std::max(1, atoi(need("--frontend-threads")));
         else if (s == "--sid") a.sid = atoi(need("--sid"));
         else if (s == "--length-scale") a.length_scale = (float)atof(need("--length-scale"));
+        else if (s == "--noise-scale") a.noise_scale = (float)atof(need("--noise-scale"));
+        else if (s == "--noise-scale-w") a.noise_scale_w = (float)atof(need("--noise-scale-w"));
+        else if (s == "--seed") a.seed = strtoull(need("--seed"), nullptr, 0);
         else if (s == "--selftest-wav") {
             std::vector<int16_t> tone(stts::kSampleRate);
             for (size_t n = 0; n < tone.size(); ++n) tone[n] = (int16_t)std::lrint(8000.0 * std::sin(2.0 * M_PI * 440.0 * n / stts::kSampleRate));
@@ -191,6 +210,7 @@ int main(int argc, char** argv) {
     auto add = [&](const std::string& t, int sid, float ls, const std::string& out) -> bool {
         Utt u;
         u.text = t; u.sid = sid; u.ls = ls; u.out = out;
+        u.seed = a.seed + utts.size();          // job index in input order: independent of the GPU partition below
         if (a.ids) {
             std::istringstream is(t);
             long v;
@@ -280,7 +300,7 @@ int main(int argc, char** argv) {
     std::vector<std::string> errs(G);
     std::vector<int> rcs(G, 0);
     std::vector<std::thread> th;
-    for (int g = 0; g < G; ++g) th.emplace_back([&, g] { rcs[g] = run_device(g, model, work[g], &errs[g]); });
+    for (int g = 0; g < G; ++g) th.emplace_back([&, g] { rcs[g] = run_device(g, model, work[g], a.noise_scale, a.noise_scale_w, &errs[g]); });
     for (auto& t : th) t.join();
     for (int g = 0; g < G; ++g)
         if (rcs[g]) { fprintf(stderr, "tts_b200: %s\n", errs[g].c_str()); return 1; }
